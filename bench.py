@@ -20,6 +20,9 @@ A "step" = one `Operator.apply` of the Forward operator over NT time steps.
              with array-valued vp/eps/delta/theta/phi, 512^3) at N=1, C5 (so=8, 2048x1024x1024 FIXED, x-slabs =
              strong scaling) at every N
 
+`--dump-outputs DIR` writes what the last timed apply returned (Bench.dump_outputs). The inputs are synthetic
+and fixed by the arguments, so two builds run with the same arguments can be compared output for output.
+
 `--impl reference` times the reference's own CPU code path (oracle/_ref = C code emitted by the
 reference's code generator for this operator, compiled here with its flags; else the oracle
 port) on the SAME grid, a bounded number of time steps per "step".
@@ -47,6 +50,7 @@ sys.path.insert(0, ROOT)
 
 B_ALG = {'iso': 16.0, 'tti': 28.0,    # algorithmic bytes / point / step (SURVEY §8d)
          'tti-arrays': 52.0}           # + cx, cy, cz, 1+2eps, sqrt(1+2delta), m/dt^2 tables (DESIGN §3.3a2)
+DUMP_SAMPLE = 1 << 20                  # grid points per wavefield in the seeded sample of --dump-outputs
 
 
 def parse():
@@ -68,7 +72,12 @@ def parse():
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the C3/C4/C5 side runs')
     ap.add_argument('--no-parity', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned as DIR/<name>.npy (see dump_outputs)')
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    return a
 
 
 def peaks():
@@ -342,12 +351,13 @@ class Bench:
         u = dv.TimeFunction(name='u', grid=model.grid, time_order=2, space_order=so)
         v = dv.TimeFunction(name='v', grid=model.grid, time_order=2, space_order=so) if tti else None
         w = dict(kind=kind, so=so, model=model, geometry=geometry, solver=solver, u=u, v=v,
-                 src=geometry.src, rec=geometry.rec, nt_steps=geometry.nt - 2, dt=float(dt),
+                 src=geometry.src, rec=geometry.rec, src_x=nbl + (shape[0] - 1) // 2,
+                 nt_steps=geometry.nt - 2, dt=float(dt),
                  shape_total=tuple(shape_total), pts_step=float(np.prod(shape_total)) * (geometry.nt - 2),
                  fkw=dict(v=v) if tti else {})
         return w
 
-    def run_resident(self, w, steps, warmup, clocks=True):
+    def run_resident(self, w, steps, warmup, clocks=True, dump=None):
         L = self.L
         fn = lambda: w['solver'].forward(src=w['src'], rec=w['rec'], u=w['u'], **w['fkw'])
         for _ in range(warmup):
@@ -362,6 +372,8 @@ class Bench:
         else:
             t = self.timed(fn, steps)
             clocks = None
+        if dump:
+            self.dump_outputs(w, dump)
         launches = int(L.b2_launch_count() - launches0)
         # second pass, same applies: CUDA events around every stencil launch -> mean launch duration
         L.b2_kernel_timing_enable(1)
@@ -396,6 +408,27 @@ class Bench:
         else:
             out['roofline'] = None
         return out
+
+    def dump_outputs(self, w, d):
+        """What the last timed apply returned to its caller, as float32 `DIR/<name>.npy`: the receiver traces
+        `rec` in full and, of each wavefield (`u`, and `v` for TTI; all three time slots), the x-plane through the
+        source `<f>_plane_x` and the grid points of a fixed seeded sample `<f>_sample` (a whole field is
+        gigabytes). Under decomposition the sample is of each rank's slab (`<f>_sample_rank<r>`) and the plane
+        comes from the rank that owns it."""
+        os.makedirs(d, exist_ok=True)
+        out = {'rec': w['rec'].data_ro_domain} if self.rank == 0 else {}
+        lo, hi = w['model'].grid.distributor.x_range if self.nranks > 1 else (0, w['u'].shape[1])
+        sfx = f'_rank{self.rank}' if self.nranks > 1 else ''
+        for name in ('u', 'v'):
+            if w[name] is None:
+                continue
+            a = w[name].data_ro_domain                         # (3, x, y, z): read-only, the device copy stays valid
+            if lo <= w['src_x'] < hi:
+                out[f'{name}_plane_x'] = a[:, w['src_x'] - lo]
+            pts = np.unique(np.random.default_rng(2024 + self.rank).integers(0, np.prod(a.shape[1:]), DUMP_SAMPLE))
+            out[f'{name}_sample{sfx}'] = a[(slice(None),) + np.unravel_index(pts, a.shape[1:])]
+        for name, arr in out.items():
+            np.save(os.path.join(d, name + '.npy'), np.ascontiguousarray(arr, dtype=np.float32))
 
     def run_e2e(self, w, steps, warmup):
         u, model, src, rec = w['u'], w['model'], w['src'], w['rec']
@@ -531,7 +564,7 @@ def main():
     else:
         total = (nranks * G, G, G)                           # every rank owns a G-plane slab
     w = b.workload(a.workload, so, total, NT)
-    res = b.run_resident(w, a.steps, a.warmup)
+    res = b.run_resident(w, a.steps, a.warmup, dump=a.dump_outputs)
     halo_path = None
     if nranks > 1:
         halo_path = ("NCCL send/recv" if not getattr(w['u'].storage, 'p2p_registered', False) else

@@ -23,23 +23,22 @@ _libs = {}
 
 
 def build(fast=False):
-    target = 'liboracle_fast.so' if fast else 'liboracle.so'
-    path = os.path.join(HERE, target)
     src = os.path.join(HERE, 'oracle.c')
-    stale = not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src)
-    tag = path + '.cpu'
+    env = dict(os.environ)
+    env.pop('CC', None)
     if fast:
-        # -march=native: rebuild when the binary was made on another CPU (see refrun.cpu_signature)
-        from .refrun import cpu_signature
-        sig = cpu_signature()
-        stale = stale or not (os.path.exists(tag) and open(tag).read().strip() == sig)
-    if stale:
-        env = dict(os.environ)
-        env.pop('CC', None)
-        subprocess.run(['make', '-B', '-C', HERE, target], check=True, capture_output=True, env=env)
-        if fast:
-            with open(tag, 'w') as f:
-                f.write(sig)
+        # -march=native: built at run time for the host it runs on, outside the source tree
+        from .refrun import host_build_path
+        path = host_build_path('liboracle_fast', [src, os.path.join(HERE, 'Makefile')])
+        if not os.path.exists(path):
+            tmp = f'{path}.{os.getpid()}'
+            subprocess.run(['make', '-B', '-C', HERE, 'liboracle_fast.so', f'FAST_SO={tmp}'], check=True,
+                           capture_output=True, env=env)
+            os.replace(tmp, path)
+        return path
+    path = os.path.join(HERE, 'liboracle.so')
+    if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src):
+        subprocess.run(['make', '-B', '-C', HERE, 'liboracle.so'], check=True, capture_output=True, env=env)
     return path
 
 

@@ -41,20 +41,34 @@ def cpu_signature():
     return 'unknown'
 
 
+def host_build_path(name, sources, flags=()):
+    """Where a library compiled at run time for this host (-march=native) goes: a per-user temporary
+    directory, never the source tree, under a name keyed by the sources, the flags and the host's CPU
+    (a binary made on another CPU is never loaded)."""
+    import hashlib
+    import tempfile
+    h = hashlib.sha1()
+    for path in sources:
+        with open(path, 'rb') as f:
+            h.update(f.read())
+    h.update(' '.join(flags).encode())
+    h.update(cpu_signature().encode())
+    d = os.path.join(tempfile.gettempdir(), f'devito-b200-oracle-uid{os.getuid()}')
+    os.makedirs(d, exist_ok=True)
+    return os.path.join(d, f'{name}-{h.hexdigest()[:16]}.so')
+
+
 def _compile(name):
     src = os.path.join(REF, name + '.c')
-    so = os.path.join(REF, name + '.so')
-    tag = so + '.cpu'
     if not os.path.exists(src):
         return None
-    sig = cpu_signature()
-    built_here = os.path.exists(tag) and open(tag).read().strip() == sig
-    if not os.path.exists(so) or not built_here or os.path.getmtime(so) < os.path.getmtime(src):
-        r = subprocess.run(['gcc'] + CFLAGS + [src, '-lm', '-o', so], capture_output=True, text=True)
+    so = host_build_path(name, [src], CFLAGS)
+    if not os.path.exists(so):
+        tmp = f'{so}.{os.getpid()}'
+        r = subprocess.run(['gcc'] + CFLAGS + [src, '-lm', '-o', tmp], capture_output=True, text=True)
         if r.returncode != 0:
             return None
-        with open(tag, 'w') as f:
-            f.write(sig)
+        os.replace(tmp, so)
     try:
         return ctypes.CDLL(so)
     except OSError:

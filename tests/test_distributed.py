@@ -30,7 +30,9 @@ def _launch(args, timeout=600, extra_env=None, nproc=2):
 
 
 def test_decomposition_host_side():
-    r = _launch(['host'])
+    # both ranks stay on the host: with a device visible, a rank would bind to GPU <LOCAL_RANK>, which a
+    # machine with fewer GPUs than ranks does not have
+    r = _launch(['host'], extra_env={'CUDA_VISIBLE_DEVICES': ''})
     assert 'DIST-HOST-OK' in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
 
 
